@@ -2,10 +2,12 @@
 """bench.py -- headline benchmark: secp256k1 ECDSA verifies/s at batch 2^20 per GPU, plus (at N = 1) the
 other BASELINE.json configurations as a `workloads` object on the same JSON line.
 
-Contract (see the task's measurement section):
+Usage:
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K --warmup W   # reference CPU arm
-One JSON line on stdout from rank 0.
+One JSON line on stdout from rank 0.  Every timed loop runs exactly K steps.  --dump-outputs DIR writes what the
+timed paths returned in their last step as DIR/<name>.npy (float32), so that two builds can be compared on the same
+seeded inputs.
 
 * headline workload: BASELINE.json configs[1] -- 2^20 random (msgHash, sig, pub) triples per GPU
   (benchdata.gen_secp256k1_verify: 4096 keys, 1/64 corrupted), weak scaling: rank g verifies its own
@@ -43,6 +45,9 @@ MAC32_PER_VERIFY_REF = 301376     # BASELINE.md section 2: 2216 fm x 136 MAC32 (
 ALG_BYTES_PER_VERIFY = 161        # SURVEY 8d: e,r,s,x,y in + 1 status byte out
 LOG2_BATCH = 20
 CACHE = os.environ.get("EB200_CACHE", "/tmp/eb200_cache")
+DUMP_MAX_BYTES = 64 << 20
+DUMP_DERIVE_ROWS = 1 << 16        # fixed, seeded sample of the 2^20 derived x (all of them would be 128 MB as float32)
+DUMP_SEED = 0xE111D
 WORKLOAD = "secp256k1 batch ECDSA verify, 2^20 random sigs per GPU (BASELINE.json configs[1])"
 
 # (key, log2 n, MAC32 per unit of the REFERENCE algorithm (SURVEY 8d), algorithmic bytes per unit, seed)
@@ -188,6 +193,8 @@ def run_reference(args):
         st = c_oracle.verify_batch(ds["e"][sl], ds["r"][sl], ds["s"][sl], ds["pub"][sl], threads)
         assert np.array_equal(st, ds["expected"][sl])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"secp256k1_verify_status": st})
     value = args.steps * sample / dt
     _, one, _ = cpu_rates(ds, threads, reps=1)
     line = {
@@ -271,8 +278,9 @@ def pmap(fn, rows, wrap=None):
     return [x for part in res for x in part]
 
 
-def run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, steps, imad_peak):
-    """One of the non-headline BASELINE configurations on a single GPU."""
+def run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, steps, imad_peak, outputs=None):
+    """One of the non-headline BASELINE configurations on a single GPU.  `outputs` (a dict) receives what the
+    device-resident call returned in its last timed step."""
     import torch
     import benchdata
     n = 1 << log2n
@@ -361,14 +369,18 @@ def run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, steps, imad_pea
     torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1) / steps
     k_ms = nat.last_timing()["main_kernel_ms"]
+    if outputs is not None:
+        outputs[key + "_status"] = d_status.cpu().numpy()
+        if key == "curve25519_derive":
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_DERIVE_ROWS, replace=False))
+            outputs[key + "_x_sample"] = d_out[torch.from_numpy(rows).to(dev)].cpu().numpy()
     for _ in range(2):
         st = e2e_call()
     assert np.array_equal(st, ds["expected"]), key + ": host-buffer call differs from the generator's expectation"
     t0 = time.perf_counter()
-    e_steps = max(2, min(steps, 5))
-    for _ in range(e_steps):
+    for _ in range(steps):
         st = e2e_call()
-    e2e_dt = (time.perf_counter() - t0) / e_steps
+    e2e_dt = (time.perf_counter() - t0) / steps
     # ---- checks (outside the timed regions): oracle on >= 512 items, output bytes for derive
     verdicts = spot()
     st_np = d_status.cpu().numpy()
@@ -393,7 +405,7 @@ def run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, steps, imad_pea
     return {
         "n": n, "value": n / (ms * 1e-3), "unit": "derives/s" if key.endswith("derive") else "verifies/s",
         "ms_per_step": ms, "steps": steps, "kernel_ms": k_ms, "gen_s": round(gen_s, 1),
-        "e2e": {"value": n / e2e_dt, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": e_steps, "api": api},
+        "e2e": {"value": n / e2e_dt, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": steps, "api": api},
         "roofline": {"bound": "int32-multiplier (fma pipe)", "kernel": kernel, "achieved": ach, "peak": imad_peak,
                      "unit": "T MAC32/s", "frac": ach / imad_peak, "mac32_per_unit_reference_algorithm": mac32,
                      "hbm_gbs_algorithmic": n * alg_bytes / (k_ms * 1e-3) / 1e9},
@@ -463,12 +475,15 @@ def run_gpu(args):
     ev1.record()
     barrier()
     total_ms = ev0.elapsed_time(ev1)
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        outputs["secp256k1_verify_status"] = (gathered if world > 1 else d_status).cpu().numpy()
     # per-launch duration of the dominant kernel (events on the launch stream), last timed step
     tm_last = nat.last_timing()
     main_ms.append(tm_last["main_kernel_ms"])
     launches_per_step = tm_last["launches"]
-    # a few more individually timed launches for the roofline average
-    for _ in range(min(args.steps, 5)):
+    # as many individually timed launches again for the roofline average
+    for _ in range(args.steps):
         step()
         torch.cuda.synchronize()
         main_ms.append(nat.last_timing()["main_kernel_ms"])
@@ -495,7 +510,7 @@ def run_gpu(args):
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         return n * world * steps / float(tt.item()), tm
 
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     hp = {k: torch.from_numpy(ds[k]).pin_memory() for k in ("e", "r", "s", "pub")}
     e2e_value, e2e_tm = e2e({k: v.numpy() for k, v in hp.items()}, e2e_steps)
     e2e_pageable, _ = e2e({k: np.array(ds[k], copy=True) for k in ("e", "r", "s", "pub")}, e2e_steps)
@@ -557,9 +572,12 @@ def run_gpu(args):
                 for key, log2n, mac32, alg_bytes, seed in EXTRA:
                     if args.only and key not in args.only.split(","):
                         continue
-                    wl[key] = run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, max(3, min(args.steps, 5)), imad_peak)
+                    wl[key] = run_extra(key, log2n, mac32, alg_bytes, seed, lib, nat, dev, args.steps, imad_peak,
+                                        outputs if args.dump_outputs else None)
                     torch.cuda.empty_cache()
                 line["workloads"] = wl
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -620,6 +638,8 @@ def run_single_process(args):
             ev[g][1].record()
     sync()
     total_ms = max(ev[g][0].elapsed_time(ev[g][1]) for g in range(N))        # max over GPUs, device clocks
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"secp256k1_verify_status": np.concatenate([s.cpu().numpy() for s in d_status])})
     ms_per_step = total_ms / args.steps
     value = n * N / (ms_per_step * 1e-3)
     # ---- end-to-end arm: one host call over the whole batch, host buffers, library-internal sharding
@@ -631,7 +651,7 @@ def run_single_process(args):
         for _ in range(steps):
             st = ec.verify_batch_packed(hn["e"], hn["r"], hn["s"], hn["pub"])
         return n * N * steps / (time.perf_counter() - t0), nat.last_timing()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     hp = {k: torch.from_numpy(big[k]).pin_memory() for k in cols}
     e2e_value, tm = e2e({k: v.numpy() for k, v in hp.items()}, e2e_steps)
     e2e_pageable, _ = e2e(big, e2e_steps)
@@ -666,10 +686,27 @@ def claim_stdout():
         os.dup2(2, 1)
 
 
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy in float32 (statuses and bytes are small integers: exact)."""
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "outputs to dump: %d bytes > %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def emit(line):
     out = _JSON_OUT if _JSON_OUT is not None else sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
 
 
 def main():
@@ -681,13 +718,15 @@ def main():
         os.environ.setdefault("NCCL_DEBUG_SUBSYS", "INIT")
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-workloads", action="store_true", help="headline only (development)")
     ap.add_argument("--only", default="", help="comma-separated subset of the extra workloads (development)")
     ap.add_argument("--single-process", action="store_true",
                     help="drive all --gpus N devices from this one process through the library's own sharding")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what they returned in their last step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -72,16 +72,16 @@ __device__ __forceinline__ fe fe_sqr_cs_inl(const fe& a) { u32 t[16]; sqr_wide_c
 
 // two independent products per call: half the call marshalling per product and two carry chains to interleave
 struct fe_pair { fe a, b; };
-__device__ __noinline__ fe_pair fe_mul2(fe a, fe b, fe c, fe d) { fe_pair r; r.a = fe_mul_inl(a, b); r.b = fe_mul_inl(c, d); return r; }
-__device__ __noinline__ fe_pair fe_sqr2(fe a, fe c) { fe_pair r; r.a = fe_sqr_inl(a); r.b = fe_sqr_inl(c); return r; }
+__device__ __noinline__ fe_pair fe_mul2_call(fe a, fe b, fe c, fe d) { fe_pair r; r.a = fe_mul_inl(a, b); r.b = fe_mul_inl(c, d); return r; }
+__device__ __noinline__ fe_pair fe_sqr2_call(fe a, fe c) { fe_pair r; r.a = fe_sqr_inl(a); r.b = fe_sqr_inl(c); return r; }
 
 template <int OP>
 __global__ void k_fe2(u32* out, u32 seed) {
   fe a, b, c, d;
   for (int i = 0; i < 8; i++) { a.v[i] = seed * (i + 1) + threadIdx.x; b.v[i] = seed * (i + 7) + blockIdx.x + 3 * threadIdx.x; c.v[i] = a.v[i] ^ 0x5555; d.v[i] = b.v[i] + 77; }
   for (int it = 0; it < ITERS / 4; it++) {
-    if (OP == 0) { fe_pair r = fe_mul2(a, b, c, d); a = r.a; c = r.b; r = fe_mul2(b, a, d, c); b = r.a; d = r.b; }
-    if (OP == 1) { fe_pair r = fe_sqr2(a, c); a = r.a; c = r.b; r = fe_sqr2(b, d); b = r.a; d = r.b; }
+    if (OP == 0) { fe_pair r = fe_mul2_call(a, b, c, d); a = r.a; c = r.b; r = fe_mul2_call(b, a, d, c); b = r.a; d = r.b; }
+    if (OP == 1) { fe_pair r = fe_sqr2_call(a, c); a = r.a; c = r.b; r = fe_sqr2_call(b, d); b = r.a; d = r.b; }
     if (OP == 2) { a = fe_mul(a, b); c = fe_mul(c, d); b = fe_mul(b, a); d = fe_mul(d, c); }          // same work, four calls
     if (OP == 3) { a = fe_mul_inl(a, b); c = fe_mul_inl(c, d); b = fe_mul_inl(b, a); d = fe_mul_inl(d, c); }
   }

@@ -1,5 +1,5 @@
 """Pins the oracle (oracle/ref_py) to the reference's own fixtures and KATs (tests/golden/,
-extracted from /root/reference by tests/golden/make_golden.py) and to OpenSSL / libsodium."""
+extracted from a checkout of the reference by tests/golden/make_golden.py) and to OpenSSL / libsodium."""
 import gzip
 import hashlib
 import json
@@ -200,13 +200,14 @@ def test_op_counts_match_baseline_table():
     assert 2100 < tot / 20 < 2350, tot / 20
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/test/fixtures/sign.input"), reason="reference tree not present")
-def test_ed25519_all_1024_reference_vectors_when_reference_present():
+def test_ed25519_reference_vectors_verify_from_hex():
+    """Every 8th line of test/fixtures/sign.input (stored in tests/golden/ed25519_sign_input.json.gz), with message,
+    signature and public key passed as the hex strings the fixture holds."""
     ed = EDDSA()
-    lines = [l for l in open("/root/reference/test/fixtures/sign.input").read().split("\n") if l]
-    for ln in lines[::8]:
-        sk_pk, pk, msg, sig_msg, _ = ln.split(":")
-        assert ed.verify(msg, sig_msg[:128], pk) is True
+    data = json.load(gzip.open(os.path.join(G, "ed25519_sign_input.json.gz"), "rt"))
+    assert data["total_lines"] == len(data["vectors"]) == 1024
+    for v in data["vectors"][::8]:
+        assert ed.verify(v["msg"], v["sig"], v["pk"]) is True
 
 
 @pytest.mark.parametrize("name", ["p192", "p224", "p256", "p384", "p521", "secp256k1"])
